@@ -2,7 +2,7 @@
 """bench.py -- video-frames/s of OmniTokenizer_VQGAN encode -> codes -> decode (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg3|cfg2|cfg4|cfg5]
-                    [--math f16x3|3xtf32|fp32]
+                    [--math f16x3|3xtf32|fp32] [--dump-outputs DIR]
 
 Workload (config.workload): cfg3 = batch of 8 synthetic videos 17x256x256 (the configuration the
 metric is quoted on, BASELINE.json configs[2]); under torchrun the batch is split over ranks
@@ -293,6 +293,26 @@ def time_vq_lookup(m, M, dev, flush):
             "note": "FP32-FMA-bound (3.3 kFLOP/B): the HBM figure is reported because the metric names it, the FMA fraction binds"}
 
 
+DUMP_SAMPLE = 1 << 21      # elements: a larger output is dumped as this many seeded picks (<= 32 MB with their positions)
+
+
+def write_outputs(dirname, arrays):
+    """--dump-outputs: every tensor as DIR/<name>.npy, float32 (integer code indices as float64, exact).  A tensor of more
+    than DUMP_SAMPLE elements is written as DUMP_SAMPLE elements at flat (C-order) positions drawn with a fixed seed; the
+    positions go to DIR/<name>_index.npy.  Two arrays stay within 64 MB."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    for name, t in arrays.items():
+        if t is None:
+            continue
+        if t.numel() > DUMP_SAMPLE:
+            pos = torch.randint(t.numel(), (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values
+            np.save(os.path.join(dirname, name + "_index.npy"), pos.double().numpy())
+            t = t.reshape(-1)[pos.to(t.device)]
+        t = t.detach().cpu()
+        np.save(os.path.join(dirname, name + ".npy"), t.numpy().astype(np.float32 if t.is_floating_point() else np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -302,7 +322,14 @@ def main():
     ap.add_argument("--workload", default="cfg3", choices=sorted(WORKLOADS))
     ap.add_argument("--math", default=None, help="f16x3 | 3xtf32 | fp32 (default: OMT_MATH or the engine default)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one returned (code indices "
+                    "or VAE latents, and the reconstruction) as DIR/<name>.npy; inputs and weights are seeded, so two builds "
+                    "can be compared output for output (see write_outputs).  Under torchrun rank 0 writes its own shard")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours only")
     if args.impl == "reference":
         return run_reference(args)
     if args.math:
@@ -340,13 +367,14 @@ def main():
     gathered = {}
 
     def step(x, u8=False):
-        """u8: the reconstruction leaves as uint8 frames (vqgan_eval.py's clamp / 255 / byte conversion fused into the last kernel)"""
+        """One pass of the path; returns what its caller receives: (code indices, or VAE latents; reconstruction).
+        u8: the reconstruction leaves as uint8 frames (vqgan_eval.py's clamp / 255 / byte conversion fused into the last kernel)"""
         dec = (lambda c: m.decode_u8(c, is_image)) if u8 else (lambda c: m.decode(c, is_image))
         if vae:      # KL path: no code indices, hence no collective; decode takes the channels-last latent (omnitokenizer.py:313)
             if x.shape[0] == 0:
-                return None
+                return None, None
             z = m.encode(x, is_image)
-            return dec(z if is_image else z.permute(0, 2, 3, 4, 1))
+            return z, dec(z if is_image else z.permute(0, 2, 3, 4, 1))
         codes = m.encode(x, is_image)                       # an empty shard (B < world) returns an empty, right-shaped tensor
         pending = None
         if world > 1 and not os.environ.get("OMT_BENCH_NO_GATHER"):
@@ -354,7 +382,7 @@ def main():
         rec = None if x.shape[0] == 0 else dec(codes)
         if pending is not None:
             gathered["codes"] = pending.wait()              # every rank now holds the full (B,T',h,w) index tensor
-        return rec
+        return codes, rec
 
     def barrier():
         if world > 1:
@@ -372,13 +400,18 @@ def main():
     evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]
     barrier()
     for a, b in evs:
+        out = None                   # release the previous step's outputs first: the allocator reuses their blocks
         flush.add_(1.0)
         a.record()
-        step(x_dev)
+        out = step(x_dev)
         b.record()
     barrier()
     launches = _cabi.launch_count - n0
     t_ms = sum(a.elapsed_time(b) for a, b in evs)
+    if args.dump_outputs and rank == 0:          # codes / latents and reconstruction of the same samples: rank 0's shard
+        first, rec = out
+        write_outputs(args.dump_outputs, {"latents" if vae else "codes": first, "reconstruction": rec})
+    out = None
     # the gathered codes of the last step must be the single-GPU codes of the full batch (checked once, untimed)
     gather_ok = None
     if world > 1 and not vae and "codes" in gathered:
@@ -395,7 +428,7 @@ def main():
     out_host = [torch.empty((e - s,) + shape[1:], dtype=torch.float32).pin_memory() for _ in range(2)]
     out_host_u8 = [torch.empty((e - s, 1 if is_image else shape[2], shape[-2], shape[-1], shape[1]), dtype=torch.uint8).pin_memory()
                    for _ in range(2)]
-    e2e_steps = max(3, args.steps)
+    e2e_steps = args.steps
     main = torch.cuda.current_stream()
     s_in, s_out = torch.cuda.Stream(), torch.cuda.Stream()
     xd = [torch.empty_like(x_dev) for _ in range(2)]
@@ -414,7 +447,7 @@ def main():
                 xd[sl].copy_(x_host, non_blocking=True)
                 ev_in[sl].record(s_in)
             main.wait_event(ev_in[sl])
-            rec = step(xd[sl], u8)
+            rec = step(xd[sl], u8)[1]
             ev_used[sl].record(main)
             if rec is not None:
                 rec.record_stream(s_out)                     # allocator: the tensor is still read by the copy stream

@@ -12,12 +12,11 @@ reference's ``(b t) (h w) d`` tensor); the temporal blocks index it through the
 ``(b n) t`` view exactly the way the CUDA kernels do, so the index maps here
 (scrambled PEG, window partition, patch order) are the ones the kernels use.
 
-Pinning: tests/test_oracle.py checks every function here against the UNMODIFIED
-reference (oracle/ref_loader.py) when /root/reference is present, and against the
-committed golden vectors in tests/golden/ (made by oracle/make_golden.py from the
-reference itself) everywhere else.
+Pinning: tests/test_oracle.py checks every function here against the committed
+golden vectors in tests/golden/, which oracle/make_golden.py recorded from the
+UNMODIFIED reference itself.
 
-Reference citations are relative to /root/reference/OmniTokenizer/.
+Reference citations are relative to the reference's OmniTokenizer/ directory.
 """
 from __future__ import annotations
 

@@ -1,9 +1,7 @@
-"""TEST INFRASTRUCTURE ONLY -- imports the UNMODIFIED reference from /root/reference.
+"""TEST INFRASTRUCTURE ONLY -- imports the UNMODIFIED reference from the checkout named by $OMT_REFERENCE_ROOT.
 
-Used (a) to pin oracle/omni_oracle.py (the CPU restatement) against the real
-reference and (b) by oracle/make_golden.py to generate tests/golden/*.pt.
-/root/reference does not exist on the GPU box, so nothing that runs there may
-import this module; tests that use it are skipped when the tree is absent.
+Used by oracle/make_golden.py to record the reference's outputs as tests/golden/*.pt;
+the tests compare against those files and never import this module.
 
 Recipe follows SURVEY.md Appendix D: the packages the reference imports but the
 image lacks (pytorch_lightning, timm, fairscale, imageio) are stubbed; none of
@@ -19,11 +17,11 @@ import warnings
 import torch
 import torch.nn as nn
 
-REF_ROOT = os.environ.get("OMT_REFERENCE_ROOT", "/root/reference")
+REF_ROOT = os.environ.get("OMT_REFERENCE_ROOT", "")
 
 
 def available() -> bool:
-    return os.path.isdir(os.path.join(REF_ROOT, "OmniTokenizer"))
+    return bool(REF_ROOT) and os.path.isdir(os.path.join(REF_ROOT, "OmniTokenizer"))
 
 
 _loaded = None
@@ -42,7 +40,7 @@ def load():
     if _loaded is not None:
         return _loaded
     if not available():
-        raise RuntimeError(f"reference tree not found at {REF_ROOT}")
+        raise RuntimeError(f"reference tree not found at OMT_REFERENCE_ROOT={REF_ROOT!r} (a checkout of the reference)")
     warnings.filterwarnings("ignore")
 
     class _LM(nn.Module):  # stands in for pl.LightningModule

@@ -10,7 +10,6 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "reference: needs /root/reference (build container only)")
 
 
 @pytest.fixture(scope="session")

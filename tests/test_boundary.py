@@ -10,8 +10,8 @@ import omnitokenizer_b200 as ob
 from omnitokenizer_b200 import _cabi
 from omnitokenizer_b200 import layout as L
 from oracle import omni_oracle as oo
-from oracle import ref_loader as rl
 from oracle import weights as W
+from tests.util import load_golden
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -35,24 +35,20 @@ def test_state_dict_layout_matches_reference_checkpoint():
     assert res.unexpected_keys == ["image_discriminator.model0.0.weight"]
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not rl.available(), reason="/root/reference not present")
 def test_state_dict_and_flags_vs_live_reference():
-    ref, args = rl.make_model(perturb=False)
+    """The canonical reference model's state_dict layout (discriminator / LPIPS keys aside), the defaults of its two
+    argument parsers and its latent_shape, as recorded in tests/golden/reference_checks.pt (oracle/make_golden.py)."""
+    fx = load_golden("reference_checks")
     m = ob.OmniTokenizer_VQGAN(ob.canonical_args())
-    rsd = {k: v for k, v in ref.state_dict().items()
-           if not k.startswith(("image_discriminator", "video_discriminator", "perceptual_model"))}
+    rsd = fx["state_dict_layout"]
     msd = m.state_dict()
     assert set(rsd) == set(msd)
     for k in rsd:
-        assert rsd[k].shape == msd[k].shape and rsd[k].dtype == msd[k].dtype, k
+        assert rsd[k] == (tuple(msd[k].shape), str(msd[k].dtype)), k
     # every flag of the reference's two parsers exists with the same default
-    ot, base = rl.load()
-    rp = ot.VQGAN.add_model_specific_args(base.VQGAN.add_model_specific_args(argparse.ArgumentParser()))
     mp = ob.OmniTokenizer_VQGAN.add_model_specific_args(ob.OmniTokenizer_VQGAN.add_base_model_args(argparse.ArgumentParser()))
-    rd, md = vars(rp.parse_args([])), vars(mp.parse_args([]))
-    assert rd == md
-    assert m.latent_shape == ref.latent_shape
+    assert fx["flag_defaults"] == vars(mp.parse_args([]))
+    assert m.latent_shape == fx["latent_shape"]
 
 
 def test_module_surface():

@@ -129,3 +129,26 @@ def test_bench_reference_arm_contract():
     cb = line["cpu_baseline"]
     assert cb["kind"] == "port" and cb["cores"] >= 1 and cb["value"] == line["value"] > 0 and "full batch" in cb["sample"]
     assert line["e2e"] == {"value": line["value"], "unit": "frames/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
+
+
+def test_bench_dump_outputs_format(tmp_path):
+    """`bench.py --dump-outputs DIR`: integer codes as exact float64 in their own shape; a float32 output above DUMP_SAMPLE
+    elements as a sample at seeded flat positions (written next to it), the same positions on every run; 64 MB at most."""
+    import numpy as np
+    import bench
+    codes = torch.randint(0, 8192, (2, 5, 4, 4))
+    rec = torch.randn(2, bench.DUMP_SAMPLE // 2 + 1)
+    dumps = []
+    for d in ("a", "b"):
+        bench.write_outputs(str(tmp_path / d), {"codes": codes, "reconstruction": rec, "absent": None})
+        dumps.append({f: np.load(tmp_path / d / f) for f in sorted(os.listdir(tmp_path / d))})
+    a, b = dumps
+    assert sorted(a) == ["codes.npy", "reconstruction.npy", "reconstruction_index.npy"]
+    assert all(np.array_equal(a[f], b[f]) for f in a)
+    assert a["codes.npy"].dtype == np.float64 and np.array_equal(a["codes.npy"], codes.numpy())
+    pos = a["reconstruction_index.npy"]
+    assert a["reconstruction.npy"].dtype == np.float32 and a["reconstruction.npy"].shape == pos.shape == (bench.DUMP_SAMPLE,)
+    assert np.array_equal(a["reconstruction.npy"], rec.reshape(-1).numpy()[pos.astype(np.int64)])
+    # the largest possible dump: two sampled arrays, one of them integer codes
+    bench.write_outputs(str(tmp_path / "c"), {"codes": torch.zeros(bench.DUMP_SAMPLE + 1, dtype=torch.long), "reconstruction": rec})
+    assert sum(os.path.getsize(tmp_path / "c" / f) for f in os.listdir(tmp_path / "c")) <= 64 << 20

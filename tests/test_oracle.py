@@ -1,10 +1,9 @@
 """CPU tests: the oracle restatement vs the committed golden vectors (made by the UNMODIFIED reference,
-oracle/make_golden.py) and, when /root/reference is present, vs the reference itself."""
+oracle/make_golden.py)."""
 import pytest
 import torch
 
 from oracle import omni_oracle as oo
-from oracle import ref_loader as rl
 from oracle import weights as W
 from tests.util import check_sub, golden_setup, load_golden
 
@@ -73,24 +72,18 @@ def test_frame_count_assert():
         oo.encode(sd, cfg, torch.zeros(1, 3, 6, 64, 64))
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not rl.available(), reason="/root/reference not present (GPU box)")
 @pytest.mark.parametrize("shape", [(1, 3, 64, 64), (1, 3, 5, 64, 64)])
 def test_oracle_matches_live_reference(shape):
-    m, args = rl.make_model(perturb=False)
-    cfg = oo.Config.from_args(args)
-    sd = W.make_state_dict(cfg, 3)
-    m.load_state_dict(sd, strict=False)
-    x = W.synthetic_input(shape, 99)
+    """encode / decode of the reference itself on weight seed 3 (tests/golden/reference_checks.pt, oracle/make_golden.py)."""
+    fx = load_golden("reference_checks")["parity"][shape]
+    cfg, sd, x = golden_setup(fx)
     is_image = x.ndim == 4
     with torch.no_grad():
-        emb_r, idx_r = m.encode(x, is_image, include_embeddings=True)
-        rec_r = m.decode(idx_r, is_image)
         emb_o, idx_o = oo.encode(sd, cfg, x, include_embeddings=True)
         rec_o = oo.decode(sd, cfg, idx_o, is_image)
-    assert torch.equal(idx_r, idx_o)
-    assert (emb_r - emb_o).abs().max() < 1e-6
-    assert (rec_r - rec_o).abs().max() < 2e-5
+    assert torch.equal(fx["idx"].long(), idx_o)
+    check_sub(fx["emb"], emb_o, 1e-6, "embeddings")
+    check_sub(fx["rec"], rec_o, 2e-5, "reconstruction")
 
 
 def test_library_op_form_agrees_with_restatement():
@@ -160,46 +153,35 @@ def test_3xtf32_numerics_model_keeps_code_indices(name, monkeypatch):
     assert err["tf32"][1] > 20 * err["3xtf32"][1], err                 # the single-pass mode is far off fp32 grade
 
 
-@pytest.mark.reference
 def test_consumer_restatements_match_live_reference():
-    """SURVEY.md 8f: Net2NetTransformer.encode_to_z (lm_transformer.py:258-268) run UNBOUND on a stub carrying the live
-    reference VQGAN, against the oracle's restatement; plus shift_dim / the eval script's uint8 expression."""
-    from oracle import ref_loader as rl
-    if not rl.available():
-        pytest.skip("reference tree not present")
-    import types
-    ref, args = rl.make_model(seed=3)
-    import OmniTokenizer.lm_transformer as lt
-    from OmniTokenizer.utils import shift_dim
-    sd = {k: v.detach().clone() for k, v in ref.state_dict().items()}
-    cfg = oo.Config()
-    x = W.synthetic_input((1, 3, 9, 64, 64), 55)
+    """SURVEY.md 8f: Net2NetTransformer.encode_to_z (lm_transformer.py:258-268) run UNBOUND on a stub carrying the reference
+    VQGAN, against the oracle's restatement; plus shift_dim / the eval script's uint8 expression.  The reference's answers
+    are recorded in tests/golden/reference_checks.pt (oracle/make_golden.py)."""
+    golden = load_golden("reference_checks")
+    fx = golden["encode_to_z"]
+    cfg, sd, x = golden_setup(fx)
     for n in (0, 2):
-        stub = types.SimpleNamespace(vtokens=False, first_stage_model=ref, sample_every_n_latent_frames=n)
         with torch.no_grad():
-            emb_r, tgt_r = lt.Net2NetTransformer.encode_to_z(stub, x, False)
             emb_o, tgt_o = oo.encode_to_z(sd, cfg, x, False, n)
-        assert torch.equal(tgt_r, tgt_o) and (emb_r - emb_o).abs().max().item() < 1e-5
-    v = torch.rand(2, 3, 5, 8, 8) - 0.5
-    assert torch.equal(shift_dim(torch.clamp(v + 0.5, 0, 1) * 255, 1, -1).byte(), oo.to_u8(v))
+        assert torch.equal(fx[n]["targets"].long(), tgt_o) and (fx[n]["emb"] - emb_o).abs().max().item() < 1e-5
+    assert torch.equal(golden["eval_u8"]["u8"], oo.to_u8(golden["eval_u8"]["video"]))
 
 
-@pytest.mark.reference
 @pytest.mark.parametrize("strategy", ["average", "first"])
 def test_inflate_gen_matches_live_reference(strategy):
     """Checkpoint tooling (SURVEY.md 8f-4): omnitokenizer_b200.ckpt.inflate_gen vs OmniTokenizer/utils.py:11 on a synthetic
-    checkpoint, key for key and bit for bit; the inflated checkpoint then loads into the module without missing keys."""
-    from oracle import ref_loader as rl
-    if not rl.available():
-        pytest.skip("reference tree not present")
-    rl.load()
-    from OmniTokenizer.utils import inflate_gen as ref_inflate
+    checkpoint, key for key and bit for bit (the reference's output is recorded as, per key, "input" where it kept the input
+    tensor and a sha256 of dtype, shape and bytes elsewhere); the inflated checkpoint then loads into the module without
+    missing keys."""
     import omnitokenizer_b200 as ob
     from omnitokenizer_b200.ckpt import inflate_gen
+    from oracle.make_golden import tensor_digest
+    fx = load_golden("reference_checks")["inflate_gen"]
     sd = W.make_state_dict(oo.Config(), 4)
-    a, b = inflate_gen(sd, 4, 8, strategy), ref_inflate(sd, 4, 8, strategy=strategy)
+    assert W.fingerprint(sd) == fx["fingerprint"]
+    a, b = inflate_gen(sd, 4, 8, strategy), fx[strategy]
     assert a.keys() == b.keys()
-    assert all(torch.equal(a[k], b[k]) for k in a)
+    assert all(torch.equal(a[k], sd[k]) if b[k] == "input" else tensor_digest(a[k]) == b[k] for k in a)
     m = ob.OmniTokenizer_VQGAN(ob.canonical_args())
     res = m.load_state_dict(a, strict=False)
     assert not res.missing_keys
