@@ -153,7 +153,10 @@ int omt_attn_window(const float* q, int ldq, const float* k, int ldk, const floa
                     float scale, omt_stream_t stream);
 
 /* Temporal attention: for every (b, n) a sequence over t' (rows b*T*N + t*N + n), optional causal
- * mask (attention.py:451 is_causal); 1 <= T <= 17. */
+ * mask (attention.py:451 is_causal: key j <= query i); any T >= 1, exact fp32 on CUDA cores.
+ * T <= 17: one warp per (b, n, head) holds the whole sequence in registers (one instance per T);
+ * T > 17: one warp per (b, n, head) and tile of 32 query frames streams K / V through shared memory in
+ * chunks of 16 frames with an online softmax.  Either way a result does not depend on B, N or the grid. */
 int omt_attn_temporal(const float* q, int ldq, const float* k, int ldk, const float* v, int ldv,
                       float* o, uint16_t* o_hi, uint16_t* o_lo, int ldo, int B, int T, int N, int heads, float scale, int causal,
                       omt_stream_t stream);

@@ -247,6 +247,147 @@ static int launch_temporal(const float* q, int ldq, const float* k, int ldk, con
   return OMT_OK;
 }
 
+// Temporal attention for T' > 17: one warp per (b, n, head) and tile of 32 query frames, lane = query frame.  q and the
+// O accumulator stay in registers; K / V stream through shared memory in chunks of TK frames (cp.async, double-buffered
+// per warp, so no block barrier), and every lane reads the same k_j / v_j (a broadcast: no bank conflicts, no shuffles).
+// Online softmax per lane with one max update and one O rescale per chunk.  The arithmetic of an output element depends
+// on T', its frame and the causal flag only -- never on B, N or the grid -- so a batch shard reproduces the full batch.
+constexpr int TQ = 32;    // query frames per warp (one per lane)
+constexpr int TK = 16;    // key frames per chunk
+constexpr int TW = 4;     // warps (consecutive b*N + n sequences of one head) per CTA
+constexpr int T_WARP_FLOATS = 2 * 2 * TK * AD;          // [buffer][K | V][TK][64] per warp: 16 KiB
+constexpr int T_SMEM = TW * T_WARP_FLOATS * 4;
+
+__device__ __forceinline__ void cp_async16(float* dst, const float* src, bool ok) {    // zero-fill when !ok
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"((uint32_t)__cvta_generic_to_shared(dst)), "l"(src),
+               "r"(ok ? 16 : 0) : "memory");
+}
+
+__global__ void __launch_bounds__(TW * 32) attn_temporal_long_kernel(const float* __restrict__ q, int ldq,
+                                                                      const float* __restrict__ k, int ldk,
+                                                                      const float* __restrict__ v, int ldv,
+                                                                      float* __restrict__ o, uint16_t* __restrict__ o_hi,
+                                                                      uint16_t* __restrict__ o_lo, int ldo, int B, int T,
+                                                                      int N, float scale, int causal) {
+  pdl_sync();
+  extern __shared__ __align__(16) float tsm[];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const long long seq = (long long)blockIdx.x * TW + warp;      // b * N + n
+  if (seq >= (long long)B * N) return;                          // ragged B*N: warps never meet at a block barrier
+  const int b = (int)(seq / N), n = (int)(seq % N);
+  const size_t row0 = (size_t)b * T * N + n;                    // canonical row of frame t: row0 + t * N
+  const size_t col = (size_t)blockIdx.y * AD;
+  const int q0 = blockIdx.z * TQ, i = q0 + lane;
+  const int kend = causal ? min(T, q0 + TQ) : T;                // a causal tile stops at its last query's key
+  const int nch = (kend + TK - 1) / TK;
+  float* const sm = tsm + warp * T_WARP_FLOATS;
+
+  // chunk c -> buffer c & 1: TK rows of 256 bytes each for K and V, 16 consecutive lanes per row; frames >= kend read as 0
+  auto load = [&](int c) {
+    float* dst = sm + (c & 1) * (2 * TK * AD);
+#pragma unroll
+    for (int it = 0; it < TK * 16 / 32; ++it) {
+      const int idx = it * 32 + lane, r = idx >> 4, sg = (idx & 15) * 4;
+      const int t = c * TK + r;
+      const size_t row = row0 + (size_t)(t < kend ? t : 0) * N;
+      cp_async16(dst + r * AD + sg, k + row * ldk + col + sg, t < kend);
+      cp_async16(dst + TK * AD + r * AD + sg, v + row * ldv + col + sg, t < kend);
+    }
+    asm volatile("cp.async.commit_group;" ::: "memory");
+  };
+  load(0);
+
+  float qr[AD], acc[AD];
+  {
+    const float* qp = q + (row0 + (size_t)(i < T ? i : 0) * N) * ldq + col;
+#pragma unroll
+    for (int d = 0; d < AD; d += 4) {
+      const float4 x = *reinterpret_cast<const float4*>(qp + d);
+      qr[d] = x.x; qr[d + 1] = x.y; qr[d + 2] = x.z; qr[d + 3] = x.w;
+      acc[d] = acc[d + 1] = acc[d + 2] = acc[d + 3] = 0.f;
+    }
+  }
+  float m = -INFINITY, l = 0.f;
+  for (int c = 0; c < nch; ++c) {
+    if (c + 1 < nch) {       // buffer (c + 1) & 1 was released by the __syncwarp that ended chunk c - 1
+      load(c + 1);
+      asm volatile("cp.async.wait_group 1;" ::: "memory");
+    } else {
+      asm volatile("cp.async.wait_group 0;" ::: "memory");
+    }
+    __syncwarp();
+    const float* Kc = sm + (c & 1) * (2 * TK * AD);
+    const float* Vc = Kc + TK * AD;
+    float s[TK];
+#pragma unroll
+    for (int j = 0; j < TK; ++j) s[j] = 0.f;
+#pragma unroll
+    for (int d = 0; d < AD; d += 4)
+#pragma unroll
+      for (int j = 0; j < TK; ++j) {
+        const float4 kf = *reinterpret_cast<const float4*>(Kc + j * AD + d);
+        s[j] = fmaf(qr[d], kf.x, s[j]);
+        s[j] = fmaf(qr[d + 1], kf.y, s[j]);
+        s[j] = fmaf(qr[d + 2], kf.z, s[j]);
+        s[j] = fmaf(qr[d + 3], kf.w, s[j]);
+      }
+    // key 0 is in chunk 0 and visible to every query, so mc is finite from the first chunk on; a later chunk that is
+    // fully masked for this lane leaves corr = 1 and adds p = 0
+    float mc = m;
+#pragma unroll
+    for (int j = 0; j < TK; ++j) {
+      const int t = c * TK + j;
+      s[j] = (t < T && (!causal || t <= i)) ? s[j] * scale : -INFINITY;
+      mc = fmaxf(mc, s[j]);
+    }
+    const float corr = expf(m - mc);
+    m = mc;
+    l *= corr;
+#pragma unroll
+    for (int d = 0; d < AD; ++d) acc[d] *= corr;
+#pragma unroll
+    for (int j = 0; j < TK; ++j) {
+      const float p = expf(s[j] - mc);
+      l += p;
+#pragma unroll
+      for (int d = 0; d < AD; d += 4) {
+        const float4 vf = *reinterpret_cast<const float4*>(Vc + j * AD + d);
+        acc[d] = fmaf(p, vf.x, acc[d]);
+        acc[d + 1] = fmaf(p, vf.y, acc[d + 1]);
+        acc[d + 2] = fmaf(p, vf.z, acc[d + 2]);
+        acc[d + 3] = fmaf(p, vf.w, acc[d + 3]);
+      }
+    }
+    __syncwarp();            // every lane is done with this buffer before chunk c + 2 refills it
+  }
+  if (i >= T) return;
+  const float inv = 1.0f / l;
+  const size_t off = (row0 + (size_t)i * N) * ldo + col;
+#pragma unroll
+  for (int d = 0; d < AD; d += 4) {
+    const float4 ov = make_float4(acc[d] * inv, acc[d + 1] * inv, acc[d + 2] * inv, acc[d + 3] * inv);
+    if (o_hi != nullptr) store_split4(o_hi, o_lo, off + d, ov);
+    else *reinterpret_cast<float4*>(o + off + d) = ov;
+  }
+}
+
+static int launch_temporal_long(const float* q, int ldq, const float* k, int ldk, const float* v, int ldv, float* o,
+                                uint16_t* o_hi, uint16_t* o_lo, int ldo, int B, int T, int N, int heads, float scale,
+                                int causal, cudaStream_t st) {
+  static bool done[64];      // the attribute is per device
+  int dev = 0;
+  cudaGetDevice(&dev);
+  if (dev >= 0 && dev < 64 && !done[dev]) {
+    OMT_CUDA(cudaFuncSetAttribute(attn_temporal_long_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, T_SMEM));
+    done[dev] = true;
+  }
+  const dim3 grid((unsigned)(((long long)B * N + TW - 1) / TW), heads, (T + TQ - 1) / TQ);
+  OMT_CUDA(launch_k(attn_temporal_long_kernel, grid, dim3(TW * 32), T_SMEM, st, q, ldq, k, ldk, v, ldv, o, o_hi, o_lo, ldo,
+                    B, T, N, scale, causal));
+  OMT_LAUNCH_CHECK();
+  return OMT_OK;
+}
+
 int launch_attn_tc3(const float* q, int ldq, const float* k, int ldk, const float* v, int ldv, float* o, uint16_t* o_hi,
                     uint16_t* o_lo, int ldo, int n_seq, int N, int heads, float scale, cudaStream_t st);
 int g_attn_kernel = 3;   // N % 128 == 0: 3 = tcgen05 3xTF32, Q / P as TMEM operands (attention_tc3.cu); 1 = CUDA-core fp32
@@ -323,9 +464,13 @@ extern "C" int omt_attn_temporal(const float* q, int ldq, const float* k, int ld
   OMT_ENTER();
   int rc = check_attn_ptrs("omt_attn_temporal", q, ldq, k, ldk, v, ldv, o, o_hi, o_lo, ldo);
   if (rc) return rc;
-  OMT_REQUIRE(T >= 1 && T <= 17, "omt_attn_temporal: T'=%d unsupported (1..17)", T);
+  OMT_REQUIRE(T >= 1, "omt_attn_temporal: T'=%d unsupported (>= 1)", T);
+  OMT_REQUIRE(B >= 0 && N >= 0 && heads > 0 && heads <= 65535 && (T + TQ - 1) / TQ <= 65535 &&
+              ((long long)B * N + TW - 1) / TW <= 0x7fffffffLL, "omt_attn_temporal: grid too large");
   if ((long long)B * N == 0) return OMT_OK;
   cudaStream_t st = (cudaStream_t)stream;
+  if (T > 17)
+    return launch_temporal_long(q, ldq, k, ldk, v, ldv, o, o_hi, o_lo, ldo, B, T, N, heads, scale, causal, st);
 #define OMT_T_CASE(t) case t: return launch_temporal<t>(q, ldq, k, ldk, v, ldv, o, o_hi, o_lo, ldo, B, N, heads, scale, causal, st);
   switch (T) {
     OMT_T_CASE(1) OMT_T_CASE(2) OMT_T_CASE(3) OMT_T_CASE(4) OMT_T_CASE(5) OMT_T_CASE(6) OMT_T_CASE(7)

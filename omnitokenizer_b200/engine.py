@@ -412,7 +412,30 @@ class Engine:
                              f"{self.ws}, grid {H // self.p}x{W // self.p}): omt_attn_window is specialised for 8x8 windows")
         if ((H // self.p) * (W // self.p)) % 64 != 0:
             raise ValueError(f"tokens per frame ({(H // self.p) * (W // self.p)}) must be a multiple of 64 (attention tiles)")
-        return B, T, H, W, 1 + (T - 1) // self.pt, H // self.p, W // self.p
+        dims = B, T, H, W, 1 + (T - 1) // self.pt, H // self.p, W // self.p
+        self._check_size(*dims[4:], B)
+        return dims
+
+    # Shape limit.  Kernels index rows (and the TMA maps row coordinates) with 32-bit integers, so every buffer of a shape
+    # -- the widest is QKV at 3C fp32 per row, the video B*C*T*H*W -- must hold fewer than 2^31 elements; the spatial
+    # attention grid also takes at most 65535 frames (B*T').  Beyond that a shape is refused before anything is allocated.
+    MAX_ELEMS = 2 ** 31 - 1
+    MAX_FRAMES = 65535
+
+    def _max_batch(self, Tp: int, h: int, w: int) -> int:
+        """largest batch of T' latent frames on an h x w token grid within the shape limit"""
+        kmax = self.cin * self.pt * self.p * self.p
+        per_sample = max(Tp * h * w * max(3 * self.C, self.ku, kmax),                          # workspace rows
+                         self.cin * (1 + (Tp - 1) * self.pt) * h * self.p * w * self.p)        # the video
+        return min(self.MAX_ELEMS // per_sample, self.MAX_FRAMES // Tp)
+
+    def _check_size(self, Tp: int, h: int, w: int, B: int):
+        bmax = self._max_batch(Tp, h, w)
+        if B > bmax:
+            T, H = 1 + (Tp - 1) * self.pt, h * self.p
+            raise ValueError(f"{B} clips of {T} frames at {H}x{w * self.p} exceed the supported shape (every buffer below "
+                             f"2^31 elements, at most {self.MAX_FRAMES} latent frames per call): at most {bmax} clips of "
+                             f"this size fit; split the batch")
 
     @staticmethod
     def graphs_enabled() -> bool:
@@ -543,6 +566,7 @@ class Engine:
         Returns a fresh (B,C,T,H,W) tensor (the reference's decoder ends in .clone(), omnitokenizer.py:1116);
         with u8 = (mul, add, lo, hi, post) a fresh uint8 (B,T,H,W,C) tensor (fused consumer conversion)."""
         B, Tp, h, w = dims
+        self._check_size(Tp, h, w, B)
         ws = self._workspace(B * Tp * h * w)
         vshape = (B, self.cin, 1 + (Tp - 1) * self.pt, h * self.p, w * self.p)
         if ws.video is None or tuple(ws.video.shape) != vshape:
